@@ -5,6 +5,7 @@ Workload (configs[1]): vqvae_top.yml nets, batch 16 x 3x512x256 per GPU, codeboo
 synthetic images/masks, random-init weights.  One "step" = one forward_step over one batch.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--precision fp32|fp16] [--impl ours|reference]
+                  [--dump-outputs DIR]
 
 N>1 is launched by torchrun (one rank per GPU); the path shards over independent images (replicas,
 weak scaling), there is no data-path collective — only the timing reduction (max over ranks).
@@ -569,6 +570,24 @@ class StdoutToStderr:
         os.close(self.saved)
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, outputs):
+    """Write each output as float32 ``path/<name>.npy``.  An output larger than its share of DUMP_BYTES is written as
+    ``<name>_sample.npy``: its flattened entries at positions drawn by a fixed seed, the same positions for every run
+    of the same shapes, so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(outputs)
+    for name, t in outputs.items():
+        a = t.detach().float().cpu()
+        if a.numel() * 4 > share:
+            pick = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:share // 4].sort().values
+            a, name = a.reshape(-1)[pick], name + "_sample"
+        np.save(os.path.join(path, name + ".npy"), a.numpy())
+
+
 def emit(line):
     sys.stdout.write(json.dumps(line) + "\n")
     sys.stdout.flush()
@@ -602,6 +621,9 @@ def run():
                          "autocast analogue; fp32 = the 3-product parity mode)")
     ap.add_argument("--graph", action="store_true",
                     help="replay one captured CUDA graph per step (measured: no gain for this GPU-bound step)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (the decoded images and the "
+                         "codebook loss) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -673,6 +695,8 @@ def run():
     clk = clocks.stop() if rank == 0 else None
     launches = ops.COUNTERS["launches"] - l0
     value = world * B * args.steps / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:   # before the next step can overwrite a graph's static outputs
+        dump_outputs(args.dump_outputs, dict(dec=dec, codebook_loss=loss))
 
     # ---------------- end to end through the public API with host buffers ----------------
     x_in = torch.empty_like(xs_d[0])

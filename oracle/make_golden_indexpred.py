@@ -136,7 +136,7 @@ def main():
     out["fcn_keys"] = np.array([f"{k}:{tuple(v.shape)}" for k, v in fcn_r.state_dict().items()])
     os.makedirs(OUT, exist_ok=True)
     path = os.path.join(OUT, "index_pred.npz")
-    np.savez_compressed(path, **out)
+    R.save_golden(path, out)
     print(path, os.path.getsize(path), [tuple(d.shape) for d in dec], len(out["unet_keys"]), len(out["fcn_keys"]))
 
 

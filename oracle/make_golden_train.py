@@ -12,7 +12,6 @@ import os
 import sys
 import types
 
-import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -78,7 +77,7 @@ def main():
         out["param1/" + k] = p.detach().numpy().copy()
     os.makedirs(OUT, exist_ok=True)
     path = os.path.join(OUT, "sampler_train.npz")
-    np.savez_compressed(path, **out)
+    R.save_golden(path, out)
     print(path, os.path.getsize(path), "loss", float(loss), "vb", float(vb), "t", rec["t"].tolist(),
           "masked", int(rec["mask"].sum()))
 

@@ -5,6 +5,7 @@ from (seed, crc32(name)), so values do not depend on module construction order.
 """
 import zlib
 
+import numpy as np
 import torch
 
 
@@ -46,6 +47,34 @@ def fill_state_dict(spec, seed):
             v = 0.1 * r
         sd[key] = v.float()
     return sd
+
+
+def save_golden(path, arrays):
+    """np.savez_compressed, except that float32 arrays of 1024 entries or more are stored as their four byte planes
+    (``<name>@planes`` uint8 [4, n] and ``<name>@shape``): deflate packs the sign / exponent plane, which it cannot
+    do on interleaved float32, and the values come back bit for bit from load_golden."""
+    out = {}
+    for k, v in arrays.items():
+        v = np.asarray(v)
+        if v.dtype == np.float32 and v.size >= 1024:
+            out[k + "@planes"] = np.ascontiguousarray(v.astype("<f4").reshape(-1).view(np.uint8).reshape(-1, 4).T)
+            out[k + "@shape"] = np.array(v.shape, dtype=np.int64)
+        else:
+            out[k] = v
+    np.savez_compressed(path, **out)
+
+
+def load_golden(path):
+    """-> dict name -> array of a fixture written by save_golden"""
+    z = np.load(path)
+    out = {}
+    for k in z.files:
+        if k.endswith("@planes"):
+            name = k[:-len("@planes")]
+            out[name] = np.ascontiguousarray(z[k].T).view("<f4").reshape(tuple(z[name + "@shape"])).astype(np.float32)
+        elif not k.endswith("@shape"):
+            out[k] = z[k]
+    return out
 
 
 def spec_of(module):
@@ -136,6 +165,32 @@ TINY_VQGAN_TRAIN = dict(
 # 7e-5 of a kink -- an fp32-equivalent implementation (activation error ~1e-5) then cannot land on the other side of
 # one, which the first fixture (seed 109: a pre-activation at +1.5e-5) made a coin flip.
 VQGAN_TRAIN_AUG_SEED = 153
+
+# the reference wrapper's view of the same reduced nets (tests/test_gpu_boundary.py, oracle/make_golden_boundary.py)
+BOUNDARY_SEEDS = (("encoder", 101), ("decoder", 102), ("quant_conv", 103), ("post_quant_conv", 104), ("disc", 105))
+GRAD_SAMPLE = 256
+
+
+def boundary_opt():
+    cfg = TINY_VQGAN_TRAIN
+    e = cfg["enc"]
+    return dict(embed_dim=cfg["embed_dim"], n_embed=cfg["n_embed"], double_z=False, z_channels=e["z_channels"],
+                resolution=e["resolution"], in_channels=3, out_ch=3, ch=e["ch"], ch_mult=e["ch_mult"],
+                num_res_blocks=e["num_res_blocks"], attn_resolutions=e["attn_resolutions"], dropout=0.0,
+                n_channels=3, ndf=cfg["ndf"], disc_layers=cfg["disc_layers"], perceptual_weight=1.0,
+                disc_start_step=cfg["disc_start_step"], disc_weight_max=1.0, diff_aug=True, lr=1e-4)
+
+
+def boundary_data():
+    return dict(image=image(107, 2, 3, 64, 32), texture_mask=blocky_mask(108, 2, 64, 32, 8))
+
+
+def grad_sample_index(numel, name):
+    """fixed positions at which a fixture stores a gradient tensor: all of it up to GRAD_SAMPLE entries, else a
+    seeded choice of GRAD_SAMPLE distinct positions"""
+    if numel <= GRAD_SAMPLE:
+        return torch.arange(numel)
+    return torch.randperm(numel, generator=_gen(0, "grad_sample/" + name))[:GRAD_SAMPLE].sort().values
 
 
 # reduced index-prediction transformer for the sample_fn fixture: the reference loop hard-codes the 32x16 token grid

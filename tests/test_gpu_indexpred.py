@@ -103,7 +103,7 @@ def _mirror(unet_cfg, fcn_cfg, cuda):
 
 def test_unet_and_fcn_heads_match_reference_fixture(cuda):
     _ops()
-    gold = np.load(GOLD)
+    gold = R.load_golden(GOLD)
     u, f, _, _ = _mirror(R.TINY_UNET, R.TINY_FCN, cuda)
     x = R.latent(93, (2, R.TINY_UNET["in_channels"], 32, 16), 1.0, "feature_top").to(cuda)
     dec = u(x)

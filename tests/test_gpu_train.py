@@ -250,7 +250,7 @@ def test_train_step_matches_reference_fixture():
     from text2human_b200.transformer_train import targets_from_gt_list
     _ops()
     cfg = R.TINY_TRANSFORMER
-    gold = np.load(GOLD)
+    gold = R.load_golden(GOLD)
     net, sd, tr = _make(cfg, 71)
     x_0, gt_list, segm, tex = [t.to(DEV) if torch.is_tensor(t) else [g.to(DEV) for g in t]
                                for t in R.sampler_train_batch(72)]

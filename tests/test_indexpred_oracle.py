@@ -19,7 +19,7 @@ def _tiny_state():
 
 
 def test_restatement_matches_reference_fixture():
-    gold = np.load(GOLD)
+    gold = R.load_golden(GOLD)
     u, f, sdu, sdf = _tiny_state()
     x = R.latent(93, (2, R.TINY_UNET["in_channels"], 32, 16), 1.0, "feature_top")
     with torch.no_grad():
@@ -34,7 +34,7 @@ def test_restatement_matches_reference_fixture():
 
 def test_mirror_keeps_the_checkpoint_abi_of_the_real_size_nets():
     from text2human_b200.index_pred_arch import MultiHeadFCNHead, UNet
-    gold = np.load(GOLD)
+    gold = R.load_golden(GOLD)
     u, f = UNet(**R.REAL_UNET), MultiHeadFCNHead(**R.REAL_FCN)
     assert [f"{k}:{tuple(v.shape)}" for k, v in u.state_dict().items()] == list(gold["unet_keys"])
     assert [f"{k}:{tuple(v.shape)}" for k, v in f.state_dict().items()] == list(gold["fcn_keys"])

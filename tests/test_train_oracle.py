@@ -17,7 +17,7 @@ def _setup():
     cfg = R.TINY_TRANSFORMER
     net = TransformerMultiHead(**cfg)
     sd = R.fill_state_dict(R.spec_of(net), 71)
-    return cfg, net, sd, R.sampler_train_batch(72), np.load(GOLD)
+    return cfg, net, sd, R.sampler_train_batch(72), R.load_golden(GOLD)
 
 
 def test_train_loss_restatement_matches_reference_fixture():
